@@ -5,7 +5,7 @@ batch 256/GPU").
 
     python bench.py --gpus N --steps K --warmup W            # this repo (N>1: run under torchrun, or
                                                              #  bench.py re-launches itself with the local launcher)
-    python bench.py --impl reference --gpus N ...            # the reference's unmodified script (baseline/_ref)
+    python bench.py --impl reference --gpus N ...            # the reference's unmodified script (oracle/_ref, staged by build())
 
 Prints ONE JSON line on rank 0.  Timed region = exactly K full training steps (forward, loss,
 backward, fused allreduce + SGD update) between barrier + cuda.synchronize on both sides, CUDA events
@@ -14,6 +14,11 @@ exceeds the 126 MB L2, so no explicit L2 flush is needed ("l2": "working_set_exc
 ``e2e`` repeats the measurement through the public API with, every step, a host->device copy of that
 step's inputs from pinned memory (uint8 NHWC images, the decoded-JPEG format, + int64 labels) and a
 device->host read of the step's loss.
+
+``--dump-outputs DIR`` writes, after the K timed steps (before ``e2e`` trains on), what the last timed step handed
+back on rank 0 as float32 ``.npy`` files (see ``dump_outputs``).  Model init and the synthetic batch are seeded, so
+two builds run with the same arguments can be compared output for output.  The bf16 step is not bit-reproducible
+(fp32 atomics order: profiles/step_reproducibility.md), so compare against the spread of two runs of the same build.
 """
 from __future__ import annotations
 
@@ -28,7 +33,7 @@ import time
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, HERE)
 
-REF_SCRIPT = os.path.join(HERE, "baseline", "_ref", "PyTorch_benchmark", "src", "pytorch_synthetic_benchmark.py")
+REF_SCRIPT = os.path.join(HERE, "oracle", "_ref", "pytorch_synthetic_benchmark.py")      # oracle/reference.py
 METRIC = "resnet50_synthetic_train_images_per_sec"
 
 
@@ -46,7 +51,43 @@ def parse():
                    help="N>1: skip the engine self-checks that run before the timed region")
     p.add_argument("--cuda-graph", choices=["on", "off"], default=os.environ.get("DDL_BENCH_GRAPH", "on"),
                    help="replay the whole training step from one captured CUDA graph (falls back to eager if capture fails)")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="write the loss and updated weights of the last timed step to DIR/<name>.npy")
+    a = p.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        p.error("--steps must be >= 1 and --warmup >= 0")
+    if a.impl == "reference" and a.warmup < 1:
+        p.error("--impl reference times from the end of the last warm-up step: --warmup must be >= 1")
+    if a.impl == "reference" and a.dump_outputs:
+        p.error("--dump-outputs applies to this repo's arm only, not --impl reference")
+    return a
+
+
+DUMP_WEIGHT_SAMPLES = 1 << 22       # 16 MiB of float32; ResNet-50 has 25.6 M weights (102 MB)
+
+
+def dump_outputs(session, out_dir: str) -> None:
+    """Write what ``session.step()`` hands back to a caller, as float32 ``out_dir/<name>.npy``:
+
+    * ``loss``: the last step's loss (0-d);
+    * ``weights``: the updated fp32 master weights, every parameter flattened in ``model.parameters()`` order; above
+      ``DUMP_WEIGHT_SAMPLES`` elements, the elements at a fixed sorted sample of indices (numpy seed 0);
+    * ``bn_stats``: every floating-point buffer (BatchNorm running means / variances) flattened in ``model.buffers()``
+      order."""
+    import numpy as np
+    import torch
+
+    session.sync()
+    w = torch.cat([p.detach().reshape(-1).float() for p in session.model.parameters()])
+    if w.numel() > DUMP_WEIGHT_SAMPLES:
+        idx = np.sort(np.random.default_rng(0).choice(w.numel(), DUMP_WEIGHT_SAMPLES, replace=False))
+        w = w[torch.from_numpy(idx).to(w.device)]
+    bufs = [b.detach().reshape(-1).float() for b in session.model.buffers() if b.is_floating_point()]
+    out = {"loss": session.last_loss.detach().float().reshape(()), "weights": w,
+           "bn_stats": torch.cat(bufs) if bufs else torch.zeros(0)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy().astype(np.float32))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -200,6 +241,10 @@ def run_ours(a):
     clocks = sampler.stop() if rank == 0 else {}
     loss = float(session.last_loss)
     value = world * B * a.steps / (ms / 1e3)
+    if a.dump_outputs:
+        if rank == 0:
+            dump_outputs(session, a.dump_outputs)
+        dist.barrier()                 # the other ranks enter the e2e region's collectives only once rank 0 is done
 
     # ---- end to end: per-step H2D of the inputs from pinned memory + D2H of the loss --------------
     e2e = None
@@ -306,17 +351,11 @@ def run_ours(a):
 # ------------------------------------------------------------------------------------------------
 def run_reference(a):
     def unavailable(why):
-        if int(os.environ.get("RANK", "0")) == 0:
-            print(json.dumps({"impl": "reference", "unavailable": why}), flush=True)
-        return 0
+        print(f"bench.py --impl reference: {why}", file=sys.stderr, flush=True)
+        return 1
 
     if not os.path.isfile(REF_SCRIPT):
-        inst = os.path.join(HERE, "baseline", "install_reference.py")
-        if int(os.environ.get("RANK", "0")) == 0 and os.path.isfile(inst):
-            subprocess.run([sys.executable, inst], capture_output=True)
-        time.sleep(1.0)
-    if not os.path.isfile(REF_SCRIPT):
-        return unavailable("reference is a cookiecutter template (not pip-installable) and baseline/_ref scripts are absent")
+        return unavailable(f"{REF_SCRIPT} is missing; build() stages it from an upstream checkout (oracle/reference.py)")
     try:
         import torch
         import torchvision  # noqa: F401
@@ -353,9 +392,8 @@ def run_reference(a):
     ev = hvd.STEP_EVENTS
     if len(ev) < a.warmup + a.steps:
         return unavailable(f"reference ran {len(ev)} steps, expected {a.warmup + a.steps}")
-    first = ev[a.warmup - 1] if a.warmup > 0 else ev[0]
-    ms = first.elapsed_time(ev[a.warmup + a.steps - 1])
-    steps = a.steps if a.warmup > 0 else a.steps - 1
+    ms = ev[a.warmup - 1].elapsed_time(ev[a.warmup + a.steps - 1])      # the K steps after the last warm-up step
+    steps = a.steps
     t = torch.tensor([ms], device="cuda")
     if world > 1:
         torch.distributed.all_reduce(t, op=torch.distributed.ReduceOp.MAX)

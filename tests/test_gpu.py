@@ -91,6 +91,28 @@ def test_bench_contract_small():
     assert out["e2e"]["h2d_bytes_per_step"] == 32 * 224 * 224 * 3 + 32 * 8
 
 
+def test_bench_dump_outputs(tmp_path):
+    """--dump-outputs: the loss and (sampled) updated weights of the last timed step, float32, at most 64 MB."""
+    import numpy as np
+
+    def bench(steps, d):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", str(steps), "--warmup", "1",
+                            "--batch-size", "16", "--no-e2e", "--dump-outputs", str(d)],
+                           cwd=ROOT, capture_output=True, text=True, timeout=900)
+        assert r.returncode == 0, (r.stdout + r.stderr)[-3000:]
+        return json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1])
+
+    d = tmp_path / "dump"
+    out, out4 = bench(2, d), bench(4, tmp_path / "dump4")
+    # --steps sets the number of timed steps: the timed region's kernel launches double from 2 to 4 steps
+    assert out["steps"] == 2 and out["gpu_launches"] > 0 and out4["gpu_launches"] == 2 * out["gpu_launches"]
+    a = {f[:-4]: np.load(d / f) for f in sorted(os.listdir(d))}
+    assert sorted(a) == ["bn_stats", "loss", "weights"] and all(v.dtype == np.float32 for v in a.values())
+    assert sum((d / f).stat().st_size for f in os.listdir(d)) <= 64 << 20
+    assert float(a["loss"]) == pytest.approx(out["final_loss"], rel=1e-6)
+    assert a["weights"].size == 1 << 22 and np.isfinite(a["weights"]).all() and np.isfinite(a["bn_stats"]).all()
+
+
 def _launch(module, argv, gpus, env=None, timeout=900):
     import io
 
